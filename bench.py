@@ -6,6 +6,7 @@
                                                             # path on the host cores (see below), rank 0 only
   python bench.py --benchmark MT10 | ML45-train | ML45-test --envs-per-gpu 8192 ...   # BASELINE configs 3 and 5
   python bench.py --gather ...                               # + optional NCCL gather of obs/reward/flags (config 4)
+  python bench.py --dump-outputs DIR ...                     # + what the last timed step returned, as DIR/<name>.npy
 
 A "step" is one VectorEnv.step over all environments of a rank (4096 by default): per env 5 physics substeps
 + 1 forward pass + obs + reward + autoreset.
@@ -238,6 +239,26 @@ def run_reference(args):
 
 
 # ----------------------------------------------------------------------------- GPU arm
+DUMP_LIMIT_BYTES = 64 * 1024 * 1024
+
+
+def dump_outputs(path, outputs):
+    """Writes the tensors `env.step_torch` returned (obs, reward, terminated, truncated, info) as float32 .npy files, so
+    that two builds run with the same arguments can be compared output for output.  Above DUMP_LIMIT_BYTES a fixed,
+    seeded sample of env rows is written instead, and its row indices as env_index.npy."""
+    host = {k: v.float().cpu().numpy() for k, v in outputs.items()}
+    n = len(next(iter(host.values())))
+    row_bytes = sum(a[0].nbytes for a in host.values())
+    if n * row_bytes > DUMP_LIMIT_BYTES:
+        k = (DUMP_LIMIT_BYTES - 4096) // (row_bytes + 8)       # room for the float64 index and the .npy headers
+        rows = np.sort(np.random.default_rng(0).choice(n, k, replace=False))
+        host = {k: a[rows] for k, a in host.items()}
+        host["env_index"] = rows.astype(np.float64)
+    os.makedirs(path, exist_ok=True)
+    for k, a in host.items():
+        np.save(os.path.join(path, k + ".npy"), a)
+
+
 def build_env(args, rank, local):
     from metaworld_b200.vector_env import MetaWorldVecEnv
     from metaworld_b200 import benchmarks as B
@@ -337,7 +358,7 @@ def run_ours(args):
     setup_s = time.perf_counter() - t0
     sampler = ClockSampler(local); sampler.start()
     # ---- e2e through the numpy API: pinned H2D of actions, D2H of obs/reward/flags/info inside the timed region
-    Ke = max(3, min(K, args.e2e_steps))
+    Ke = min(K, args.e2e_steps)
     a_host = (np.random.default_rng(args.seed + rank).uniform(-1, 1, size=(Ke + 2, N, 4))).astype(np.float32)
     for i in range(2):
         env.step(a_host[i])
@@ -398,6 +419,8 @@ def run_ours(args):
     sampler.end()
     if ncu_range:
         torch.cuda.profiler.stop()
+    if args.dump_outputs and rank == 0:      # before the profiled pass below overwrites the step buffers
+        dump_outputs(args.dump_outputs, dict(obs=o, reward=r, terminated=te, truncated=tr, info=inf))
     if world > 1:
         dist.barrier()
     ms = sum(a.elapsed_time(b) for a, b in ev)
@@ -508,7 +531,11 @@ def main():
     ap.add_argument("--cpu-steps-per-env", type=int, default=600)
     ap.add_argument("--ref-steps-per-env", type=int, default=1000)
     ap.add_argument("--gather", action="store_true", help="also all-gather obs/reward/flags across ranks every step (BASELINE config 4)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write obs / reward / terminated / truncated / info of the last timed "
+                                                          "step (rank 0) as DIR/<name>.npy, float32")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0 or args.e2e_steps < 1:
+        ap.error("--steps and --e2e-steps must be >= 1 and --warmup >= 0")
     if args.impl == "reference":
         run_reference(args)
     else:

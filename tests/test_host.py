@@ -213,3 +213,27 @@ def test_bench_helpers():
     b = bench.algorithmic_bytes(["reach-v3"])
     assert b == 4 * (2 * 16 + 4 * 15 + 120)          # nq 16, nv 15 -> 848 B per env step
     assert abs(bench.algorithmic_bytes(names) - 792.32) < 0.5
+
+
+def test_bench_dump_outputs(tmp_path, monkeypatch):
+    """--dump-outputs: every step_torch output as float32 .npy; above the size cap a seeded sample of env rows (the
+    same rows every run) plus their indices, all within the cap."""
+    import importlib.util
+    import torch
+    spec = importlib.util.spec_from_file_location("bench", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    g = torch.Generator().manual_seed(0)
+    out = dict(obs=torch.rand(1000, 89, generator=g), reward=torch.rand(1000, generator=g), terminated=torch.zeros(1000, dtype=torch.uint8),
+               truncated=torch.ones(1000, dtype=torch.uint8), info=torch.rand(1000, 7, generator=g))
+    bench.dump_outputs(str(tmp_path / "full"), out)
+    for k, v in out.items():
+        a = np.load(tmp_path / "full" / f"{k}.npy")
+        assert a.dtype == np.float32 and np.array_equal(a, v.float().numpy())
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 50_000)
+    for d in ("s1", "s2"):
+        bench.dump_outputs(str(tmp_path / d), out)
+        assert sum(f.stat().st_size for f in (tmp_path / d).iterdir()) <= 50_000
+    rows = np.load(tmp_path / "s1" / "env_index.npy")
+    assert np.array_equal(rows, np.load(tmp_path / "s2" / "env_index.npy")) and 0 < len(rows) < 1000
+    assert np.array_equal(np.load(tmp_path / "s1" / "obs.npy"), out["obs"].numpy()[rows.astype(int)])

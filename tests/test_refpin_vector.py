@@ -1,24 +1,38 @@
 """CPU suite: the REAL host code of `metaworld_b200` (benchmarks.make_tasks, MetaWorldVecEnv, evaluation) against the
-REFERENCE's whole vector stack -- `gym.make_vec("Meta-World/MT10" | "ML10-train", ...)` from /root/reference running
-unmodified on oracle/refshim (gymnasium + mujoco stand-ins, see oracle/refshim/README.md).  Both sides step the same
-float64 oracle physics (ours through tests/oracle_engine.py), so every difference is host logic: goal generation, task
-selection streams, one-hot ids, TimeLimit / terminate-on-success, SAME_STEP autoreset, final_obs / final_info /
-episode statistics, checkpoint format.  Needs /root/reference, i.e. runs in the build container, not on the GPU box."""
+REFERENCE's whole vector stack -- `gym.make_vec("Meta-World/MT10" | "ML10-train", ...)` from the reference package
+running unmodified on oracle/refshim (gymnasium + mujoco stand-ins, see oracle/refshim/README.md).  Both sides step the
+same float64 oracle physics (ours through tests/oracle_engine.py), so every difference is host logic: goal generation,
+task selection streams, one-hot ids, TimeLimit / terminate-on-success, SAME_STEP autoreset, final_obs / final_info /
+episode statistics, checkpoint format.
+
+The reference is not part of this repository: what it returned to each test is stored under tests/golden/refstack/ and
+replayed (tests/refreplay.py).  tests/golden/make_refstack_goldens.py re-records it from a reference checkout."""
 import os
+import types
 
 import numpy as np
 import pytest
 
-pytestmark = pytest.mark.skipif(not os.path.isdir("/root/reference/metaworld"), reason="/root/reference not present")
 KEYS = ("success", "near_object", "grasp_success", "grasp_reward", "in_place_reward", "obj_to_target", "unscaled_reward")
+RECORD_FROM = os.environ.get("MW_REFSTACK_RECORD")      # a reference checkout: run it live and rewrite the recordings
 
 
-@pytest.fixture(scope="module")
-def gym():
-    from oracle import refshim
-    refshim.activate()
-    import gymnasium
-    return gymnasium
+@pytest.fixture
+def ref(request):
+    """`ref.gym` / `ref.metaworld`: the reference's gymnasium registry and metaworld package."""
+    from refreplay import Session
+    name = request.node.name.replace("[", "-").replace("]", "")
+    if RECORD_FROM:
+        from oracle import refshim
+        metaworld = refshim.activate(RECORD_FROM)
+        import gymnasium
+        session = Session()
+        yield session.root(types.SimpleNamespace(gym=gymnasium, metaworld=metaworld))
+        session.save(name)
+    else:
+        session = Session.load(name)
+        yield session.root()
+        session.finish()
 
 
 def _ours(kind, name, **kw):
@@ -69,7 +83,8 @@ def _compare_rollout(ref, ours, steps, seed, atol=2e-6):
     return n_done
 
 
-def test_mt10_one_hot_random_select_matches_reference_stack(gym):
+def test_mt10_one_hot_random_select_matches_reference_stack(ref):
+    gym = ref.gym
     kw = dict(seed=42, use_one_hot=True, max_episode_steps=9, terminate_on_success=True, num_goals=3)
     ref = gym.make_vec("Meta-World/MT10", vector_strategy="sync", **kw)
     ours = _ours("mt", "MT10", **kw)
@@ -82,8 +97,8 @@ def test_mt10_one_hot_random_select_matches_reference_stack(gym):
     for tr, to in zip(ref.get_attr("tasks"), ours.get_attr("tasks")):
         assert len(tr) == len(to) == 3
         for a, b in zip(tr, to):
-            import pickle
-            assert np.array_equal(pickle.loads(a.data)["rand_vec"], b.unpack()["rand_vec"]) and a.env_name == b.env_name
+            from refreplay import unpickle
+            assert np.array_equal(unpickle(a.data)["rand_vec"], b.unpack()["rand_vec"]) and a.env_name == b.env_name
     assert _compare_rollout(ref, ours, 30, seed=1) >= 30
     # evaluation protocol pieces used by metaworld/evaluation.py
     ref.call("toggle_terminate_on_success", False); ours.call("toggle_terminate_on_success", False)
@@ -100,8 +115,9 @@ def test_mt10_one_hot_random_select_matches_reference_stack(gym):
     _compare_rollout(ref, ours, 12, seed=3)
 
 
-def test_ml10_train_pseudorandom_partially_observable_matches_reference_stack(gym):
-    import metaworld
+def test_ml10_train_pseudorandom_partially_observable_matches_reference_stack(ref):
+    gym = ref.gym
+    metaworld = ref.metaworld
     kw = dict(seed=7, meta_batch_size=20, max_episode_steps=8)
     metaworld._N_GOALS = 4          # the ML entry points do not take num_goals (metaworld/__init__.py:631-654)
     ref = gym.make_vec("Meta-World/ML10-train", vector_strategy="sync", **kw)
@@ -123,9 +139,10 @@ def test_ml10_train_pseudorandom_partially_observable_matches_reference_stack(gy
 @pytest.mark.parametrize("extra", [dict(reward_normalization_method="gymnasium", normalize_observations=True),
                                    dict(recurrent_info_in_obs=True, normalize_observations=True, reward_normalization_method="exponential"),
                                    dict(recurrent_info_in_obs=True, normalize_reward_in_recurrent_info=False, reward_normalization_method="gymnasium")])
-def test_normalisation_and_recurrent_wrappers_match_reference_stack(gym, extra):
+def test_normalisation_and_recurrent_wrappers_match_reference_stack(ref, extra):
     """The non-default per-sub-env wrappers of metaworld/__init__.py:437-446, autoresets included (the observation
     statistics see the terminal AND the reset observation of a finished env; the discounted return survives truncation)."""
+    gym = ref.gym
     kw = dict(seed=11, use_one_hot=True, max_episode_steps=7, terminate_on_success=True, num_goals=2, **extra)
     ref = gym.make_vec("Meta-World/MT10", vector_strategy="sync", **kw)
     ours = _ours("mt", "MT10", **kw)
@@ -136,8 +153,8 @@ def test_normalisation_and_recurrent_wrappers_match_reference_stack(gym, extra):
     assert _compare_rollout(ref, ours, 25, seed=4, atol=3e-4) >= 30
 
 
-def test_mt1_single_task_vector_and_explicit_resets(gym):
-    import metaworld
+def test_mt1_single_task_vector_and_explicit_resets(ref):
+    metaworld = ref.metaworld
     kw = dict(seed=3, max_episode_steps=6)
     metaworld._N_GOALS = 5
     # MT1 through the reference returns the single (wrapped) env of make_mt_envs; compare through our 1-env vector view
@@ -157,11 +174,11 @@ def test_mt1_single_task_vector_and_explicit_resets(gym):
         assert np.array_equal(renv.unwrapped._last_rand_vec, ours.get_attr("_last_rand_vec")[0])
 
 
-def test_wrapped_single_env_across_truncations(gym):
+def test_wrapped_single_env_across_truncations(ref):
     """gym.make("Meta-World/MT1") form (single=True): the TimeLimit step returns the terminal observation, stepping again
     raises, and reset() starts the task the reference's RandomTaskSelectWrapper draws -- three episodes, with and without
     the optional per-env wrappers (recurrent observation + exponential reward normalisation)."""
-    import metaworld
+    metaworld = ref.metaworld
     metaworld._N_GOALS = 5
     for extra in ({}, dict(recurrent_info_in_obs=True, normalize_reward_in_recurrent_info=True), dict(use_one_hot=False, reward_normalization_method="exponential")):
         kw = dict(seed=11, max_episode_steps=5, **extra)
@@ -183,10 +200,10 @@ def test_wrapped_single_env_across_truncations(gym):
             assert np.array_equal(renv.unwrapped._last_rand_vec, ours._last_rand_vec)
 
 
-def test_bare_single_env_surface_matches_reference_class(gym):
+def test_bare_single_env_surface_matches_reference_class(ref):
     """`mt1.train_classes[name]()` + set_task / reset / step / evaluate_state and the attributes the reference's own tests
     read (tests/integration/test_new_api.py:18-45, tests/metaworld/envs/mujoco/sawyer_xyz/test_sawyer_xyz_env.py)."""
-    import metaworld
+    metaworld = ref.metaworld
     from metaworld_b200 import benchmarks as B
     from metaworld_b200.single_env import SawyerXYZEnvB200
     from oracle_engine import OracleEngine
@@ -224,8 +241,8 @@ def test_bare_single_env_surface_matches_reference_class(gym):
         oenv.step(np.zeros(3, np.float32))
 
 
-def test_goal_hidden_and_observable_envs_draw_the_reference_goal(gym):
-    import gymnasium
+def test_goal_hidden_and_observable_envs_draw_the_reference_goal(ref):
+    gymnasium = ref.gym
     from metaworld_b200.single_env import make_goal_env
     from oracle_engine import OracleEngine
     for observable, rid in ((False, "Meta-World/goal_hidden"), (True, "Meta-World/goal_observable")):
@@ -237,8 +254,9 @@ def test_goal_hidden_and_observable_envs_draw_the_reference_goal(gym):
         assert np.abs(x1[0] - x2[0]).max() < 2e-6 and (not x1[0][36:].any()) == (not observable)
 
 
-def test_custom_mt_and_ml_entry_points_match_reference(gym):
-    import metaworld
+def test_custom_mt_and_ml_entry_points_match_reference(ref):
+    gym = ref.gym
+    metaworld = ref.metaworld
     from metaworld_b200 import vector_env as V
     from oracle_engine import OracleEngine
     metaworld._N_GOALS = 3
@@ -255,9 +273,10 @@ def test_custom_mt_and_ml_entry_points_match_reference(gym):
     assert _compare_rollout(ref, ours, 14, seed=8) >= 8
 
 
-def test_every_reference_id_has_an_entry_point(gym):
+def test_every_reference_id_has_an_entry_point(ref):
     """The ids the reference registers (metaworld/__init__.py:607-820) == the ids this package registers, and the entry
     points take the reference's argument names."""
+    gym = ref.gym
     import metaworld_b200 as M
     from oracle_engine import OracleEngine
     ref_ids = {k.split("/", 1)[1] for k in gym.registry if k.startswith("Meta-World/")}
